@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run, one rank per GPU)
   python bench.py --impl reference ...                     (the CPU path timed on the host cores; rank 0 only)
+  python bench.py ... --dump-outputs DIR                   (also write what the last timed step returned, DIR/<name>.npy)
 
 One "step" = one pass of the hot path (ORB + LSD/LBD extraction of both images, L/R stereo association,
 frame-to-frame tracking, robust Gauss-Newton pose) over one batch of B consecutive synthetic stereo pairs of a
@@ -180,6 +181,42 @@ def measured_peaks():
     return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
 
 
+DUMP_FRAMES = 16            # frames of the last batch whose features --dump-outputs writes (fixed, seeded sample)
+DUMP_MAX_BYTES = 64 << 20
+
+
+def collect_outputs(fe, results, poses, B, all_poses=None):
+    """What this rank's caller of the timed path receives for its last step, as float32 / float64 arrays: every field
+    of the per-frame results (plf_batch_download), the device-resident poses (plf_batch_device_poses; with more than
+    one rank also the all-gathered poses of every rank, rank-major, as device_poses_all_ranks) and the stereo features
+    (plf_get_frame) of DUMP_FRAMES frames drawn with a fixed seed, concatenated in frame order with their counts.
+    Call before anything else runs a batch: plf_get_frame reads the last one."""
+    out = {f"result_{f}": results[f].astype(np.float64) for f in results.dtype.names}
+    out["device_poses"] = poses.cpu().numpy().astype(np.float64)
+    if all_poses is not None:
+        out["device_poses_all_ranks"] = all_poses.cpu().numpy().astype(np.float64)
+    frames = np.sort(np.random.default_rng(0).choice(B, size=min(DUMP_FRAMES, B), replace=False))
+    feats = [fe.get_frame(int(k)) for k in frames]
+    out["features_frame"] = frames.astype(np.float64)
+    out["features_n_pt"] = np.array([len(f["pt_pl"]) for f in feats], np.float64)
+    out["features_n_ls"] = np.array([len(f["ls_spl"]) for f in feats], np.float64)
+    for name in feats[0]:
+        a = np.concatenate([f[name] for f in feats])
+        out[f"features_{name}"] = a.astype(np.float32 if a.dtype in (np.uint8, np.float32) else np.float64)
+    return out
+
+
+def write_outputs(d, arrays):
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total / 2**20:.1f} MB (limit {DUMP_MAX_BYTES >> 20} MB)")
+    d = Path(d)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(d / f"{name}.npy", a)
+    print(f"bench.py: wrote {len(arrays)} arrays ({total / 2**20:.1f} MB) to {d}", file=sys.stderr)
+
+
 def cpu_baseline_run(n_frames, threads=None):
     """(pairs/s, worker processes, seconds) of the CPU path on n_frames rendered pairs; the worker pool is started
     before the clock and one untimed pass warms it up."""
@@ -253,7 +290,12 @@ def main():
     ap.add_argument("--pool", type=int, default=24, help="distinct rendered frames (ping-ponged to fill a batch)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--overlap-profile", action="store_true", help="also report per-kernel times measured with two batches in flight (overlapped)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (per-frame results, device poses, the features "
+                         "of a fixed sample of frames) as DIR/<name>.npy; the inputs depend only on the arguments")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     select_config(args.config)
     rank = int(os.environ.get("RANK", "0")); local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -349,7 +391,7 @@ def main():
             fe.batch_run(B)
         for _ in range(depth):
             gather_poses()
-            fe.batch_download_array(B)
+            last_res = fe.batch_download_array(B)
         ext.wait_stream(side)                   # the last pose exchange is inside the timed region
         e1.record(ext)
     barrier()
@@ -361,6 +403,8 @@ def main():
         timeline = [[[round(float(x), 2) for x in ph] for ph in b] for b in fe.debug_timeline()]
     except Exception:
         timeline = None
+
+    dumped = collect_outputs(fe, last_res, pose_buf, B, gather_buf) if args.dump_outputs and rank == 0 else None
 
     # ---- `e2e`: pinned host buffers -> plf_batch_upload + run + pose exchange + download, K steps
     # (software-pipelined like a streaming caller: the H2D of batch i+1 is issued while batch i runs; every step still
@@ -463,6 +507,8 @@ def main():
                     kernels=ktab)
         if overlapped:
             line["kernels_overlapped"] = overlapped
+        if dumped is not None:
+            write_outputs(args.dump_outputs, dumped)
         if world == 1 and not args.no_cpu_baseline:
             n_cpu = 48                         # ~12 s of single-core CPU work (0.25 s per pair)
             v, c, dt = cpu_baseline_run(n_cpu, None)

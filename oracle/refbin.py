@@ -1,10 +1,12 @@
 """TEST INFRASTRUCTURE.  ctypes access to oracle/_ref/liblinedesc_ref.so: the reference's own vendored
 3rdparty/line_descriptor (LSDDetectorC::detect, BinaryDescriptor::compute) and src/mapFeatures.cpp (MapPoint), compiled
-UNMODIFIED from /root/reference by
+UNMODIFIED from the reference source tree (reference_dir()) by
 oracle/ref_build/Makefile against a stand-in for the OpenCV API whose primitives on this path are the cv2-pinned
-restatements of oracle/*.c.  Used only to pin oracle/lbd.c (KeyLine stage + LBD) against the shipped reference code.
-The library is built where /root/reference exists and travels to the GPU box; available() is False otherwise."""
+restatements of oracle/*.c.  Used only to pin oracle/lbd.c (KeyLine stage + LBD) against the shipped reference code
+(tests/golden/make_golden_refbin.py stores what it returns); available() is False where it is not built."""
 import ctypes as C
+import json
+import os
 import subprocess
 from pathlib import Path
 
@@ -17,10 +19,21 @@ _SO = _DIR / "_ref" / "liblinedesc_ref.so"
 _lib = None
 
 
+def reference_dir():
+    """The reference source tree: the PLF_REFERENCE_DIR environment variable if set, else BASELINE.json's
+    reference_path.  None where that tree is absent or cannot be read (os.path.isfile is False on a permission error,
+    where Path.exists raises)."""
+    d = os.environ.get("PLF_REFERENCE_DIR") or json.loads((_DIR.parent / "BASELINE.json").read_text()).get("reference_path")
+    if d and os.path.isfile(os.path.join(d, "3rdparty", "line_descriptor", "src", "binary_descriptor_custom.cpp")):
+        return Path(d)
+    return None
+
+
 def build():
-    """Compiles the vendored sources if the reference tree is present (no-op otherwise)."""
-    if Path("/root/reference/3rdparty/line_descriptor/src/binary_descriptor_custom.cpp").exists():
-        subprocess.run(["make", "-C", str(_DIR / "ref_build")], check=True, capture_output=True)
+    """Compiles the vendored sources if the reference tree is given (no-op otherwise)."""
+    ref = reference_dir()
+    if ref is not None:
+        subprocess.run(["make", "-C", str(_DIR / "ref_build"), f"REF={ref}"], check=True, capture_output=True)
 
 
 def available():

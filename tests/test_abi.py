@@ -1,10 +1,10 @@
 """CPU tests: the C-ABI library loads and exports every symbol include/plslam_b200.h declares,
 and fails loudly (no fallback) when no CUDA device is present."""
-import ctypes as C
+import os
 import re
+import subprocess
+import sys
 from pathlib import Path
-
-import pytest
 
 ROOT = Path(__file__).resolve().parent.parent
 
@@ -36,10 +36,18 @@ def test_struct_sizes_match(built):
 
 
 def test_no_cpu_fallback(built):
-    """Without a GPU plf_create must fail with PLF_ERR_NO_DEVICE, not silently compute on the CPU."""
-    import torch
-    import plslam_b200 as plf
-    if torch.cuda.is_available():
-        pytest.skip("GPU present; the failure path is exercised on the CPU box")
-    with pytest.raises(plf.PlfError, match="no CUDA device"):
-        plf.Frontend(device=0)
+    """Without a GPU plf_create must fail with PLF_ERR_NO_DEVICE, not silently compute on the CPU.  Checked in a child
+    process that sees no device (CUDA_VISIBLE_DEVICES=""), so that it runs on GPU machines as well."""
+    code = ("import sys\n"
+            "sys.path[:0] = sys.argv[1:]\n"
+            "import plslam_b200 as plf\n"
+            "try:\n"
+            "    plf.Frontend(device=0)\n"
+            "except plf.PlfError as e:\n"
+            "    print(e)\n"
+            "else:\n"
+            "    sys.exit('a Frontend was created without a CUDA device')\n")
+    r = subprocess.run([sys.executable, "-c", code, str(ROOT), str(ROOT / "pl-slam_b200")], capture_output=True, text=True,
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), timeout=300)
+    assert r.returncode == 0, r.stdout + r.stderr
+    assert "no CUDA device" in r.stdout

@@ -5,6 +5,8 @@ import numpy as np
 import pytest
 
 from oracle import clib, synth
+from test_refbin_pin import GOLD as REF_GOLD
+from test_refbin_pin import images as refbin_images
 
 pytestmark = pytest.mark.gpu
 GOLD = Path(__file__).parent / "golden" / "lines_v1.npz"
@@ -75,41 +77,36 @@ def test_lbd_edge_cases(fe):
 
 def test_lbd_equals_vendored_reference_code(fe):
     """CUDA LBD vs the reference's own BinaryDescriptor::compute (vendored sources compiled unmodified into
-    oracle/_ref/liblinedesc_ref.so, see oracle/refbin.py): bit-exact descriptors."""
-    from oracle import refbin
-    if not refbin.available():
-        pytest.skip("oracle/_ref/liblinedesc_ref.so not present")
+    oracle/_ref/liblinedesc_ref.so, see oracle/refbin.py; its descriptors are stored in tests/golden/refbin_v1.npz):
+    bit-exact descriptors."""
+    g = np.load(REF_GOLD)
     L, R = synth.scene_pair()
-    for img in (L, R):
+    for i, img in enumerate((L, R)):
         kl = clib.keylines_from_segments(clib.lsd(img), 1242, 375, 0.025 * 375)
         kl["class_id"] = np.arange(len(kl), dtype=np.int32)
         assert len(kl) > 300
-        assert np.array_equal(fe.lbd(img, kl), refbin.lbd(img, kl))
+        assert kl.tobytes() == g[f"kl{i}"].tobytes()       # the KeyLines the reference descriptors were computed on
+        assert np.array_equal(fe.lbd(img, kl), g[f"lbd{i}"])
 
 
 def test_cuda_lines_end_to_end_equal_vendored_reference_code(built):
     """The whole CUDA line path (LSD -> KeyLine stage -> LBD, one call: plf_detect_lines) against the reference's own
-    LSDDetectorC::detect + BinaryDescriptor::compute compiled unmodified (oracle/_ref): every KeyLine field - `angle`
-    (glibc atan2f, LSDDetector_custom.cpp:286) included - and every descriptor bit, end to end, nothing of the oracle's
-    restatement in between."""
+    LSDDetectorC::detect + BinaryDescriptor::compute compiled unmodified (oracle/_ref, outputs stored in
+    tests/golden/refbin_v1.npz): every KeyLine field - `angle` (glibc atan2f, LSDDetector_custom.cpp:286) included - and
+    every descriptor bit, end to end, nothing of the oracle's restatement in between."""
     import plslam_b200 as plf
-    from oracle import refbin
-    if not refbin.available():
-        pytest.skip("oracle/_ref/liblinedesc_ref.so not present")
-    L, R = synth.scene_pair()
-    E = synth.scene_pair(w=752, h=480, seed=9)[0]
-    S = next(iter(synth.stream(plf.KITTI_CAMERA, 1, world=synth.World(seed=7), seed=42)))[1]
+    g = np.load(REF_GOLD)
     n_ulp = 0
-    for img in (L, R, E, S):
+    for i, img in enumerate(refbin_images()):
         h, w = img.shape
         cam = dict(plf.KITTI_CAMERA, width=w, height=h)
         with plf.Frontend(camera=cam, lsd_nfeatures=0) as fe:          # keep every line, detection order
             kl, desc = fe.detect_lines(img)
-        ref_kl = refbin.keylines(img, min_length=float(np.float32(0.025)) * min(w, h))
+        ref_kl = g[f"kl{i}"]
         assert len(kl) == len(ref_kl) > 150
         for f in ref_kl.dtype.names:
             assert np.array_equal(kl[f].view(np.int32), ref_kl[f].view(np.int32)), f
-        assert np.array_equal(desc, refbin.lbd(img, ref_kl))
+        assert np.array_equal(desc, g[f"lbd{i}"])
         dy = ref_kl["endPointY"] - ref_kl["startPointY"]; dx = ref_kl["endPointX"] - ref_kl["startPointX"]
         n_ulp += int((ref_kl["angle"] != np.arctan2(dy.astype(np.float64), dx.astype(np.float64)).astype(np.float32)).sum())
     assert n_ulp > 0      # the lines do include cases where atan2f and the narrowed f64 atan2 differ

@@ -1,5 +1,6 @@
 """The C++ host shim (pl-slam_b200/cpp/stvo_shim.h: StVO::StereoFrameHandler & co. on top of the C ABI), driven by
 vo_demo = the VO part of the reference's frame loop (app/plslam_dataset.cpp:111-163)."""
+import os
 import struct
 import subprocess
 from pathlib import Path
@@ -21,14 +22,13 @@ def write_frames(path, cam, frames):
 
 
 def test_shim_builds_and_fails_loudly_without_gpu(built, tmp_path):
-    import torch
+    """Run with every device hidden (CUDA_VISIBLE_DEVICES=""), so that the failure path is checked on GPU machines too."""
     assert DEMO.exists()
     cam = dict(width=64, height=48, fx=50.0, fy=50.0, cx=32.0, cy=24.0, b=0.1)
     p = tmp_path / "f.bin"
     write_frames(p, cam, [(np.zeros((48, 64), np.uint8),) * 2])
-    r = subprocess.run([str(DEMO), str(p)], capture_output=True, text=True)
-    if not torch.cuda.is_available():
-        assert r.returncode == 2 and "no CUDA device" in r.stderr      # std::runtime_error from the handler ctor
+    r = subprocess.run([str(DEMO), str(p)], capture_output=True, text=True, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert r.returncode == 2 and "no CUDA device" in r.stderr      # std::runtime_error from the handler ctor
 
 
 @pytest.mark.gpu
